@@ -524,6 +524,7 @@ def run_ours(args):
             sampler.start()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         total, iters = 0, 0
+        st = None
         e0.record(stream)
         for _ in range(steps):
             st = align(src, out)
@@ -538,14 +539,16 @@ def run_ours(args):
             dist.all_reduce(tm, op=dist.ReduceOp.MAX)
             ms = float(tm[0])
         # with the exchange inside every iteration each rank's stats already carry the GLOBAL pair counts
-        return ms, float(total), ctx.launches - l0, clocks, iters
+        return ms, float(total), ctx.launches - l0, clocks, iters, st
 
     # device-resident leg (value) --------------------------------------------------------------------------------
-    ms_v, tot_v, launches, clocks, iters_v = timed(src_dev, out_dev, args.steps, args.warmup, not args.no_clocks)
+    ms_v, tot_v, launches, clocks, iters_v, last_v = timed(src_dev, out_dev, args.steps, args.warmup, not args.no_clocks)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_v, out_dev, p2plane)
     prof = {k: ctx.profile_get(k) for k in ("icp_search", "icp_accum", "allreduce", "query_sort", "solve", "transform_out",
                                             "voxelgrid")}
     # host-buffer leg (e2e) --------------------------------------------------------------------------------------
-    ms_e1, tot_e1, _, _, _ = timed(src_host, out_host, args.steps, max(1, args.warmup // 2), False)
+    ms_e1, tot_e1, _, _, _, _ = timed(src_host, out_host, args.steps, max(1, args.warmup // 2), False)
     ms_e, tot_e, depth = ms_e1, tot_e1, 1
     pipeline_error = None
     if world == 1 and not args.no_pipeline:
@@ -704,6 +707,31 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+DUMP_ROWS = 1_000_000
+
+
+def dump_outputs(d, st, out_dev, with_normals):
+    """What the value leg's last align() handed its caller, as .npy files in d: the final transformation, the ICP state
+    and the aligned cloud (xyz, and the normals under point-to-plane) -- all rows up to DUMP_ROWS, beyond that the same
+    seeded sample of DUMP_ROWS rows on every run, with their row numbers (32 MB at most)."""
+    import torch
+    os.makedirs(d, exist_ok=True)
+    n = int(out_dev.shape[0])
+    rows = torch.arange(n) if n <= DUMP_ROWS else torch.from_numpy(
+        np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False)))
+    cloud = out_dev[rows.to(out_dev.device)].cpu().numpy()
+    arrays = {"final_transformation": np.asarray(st["final"], dtype=np.float64),
+              "icp_state": np.array([st["converged"], st["state"], st["iterations"], st["n_correspondences"], st["mse"],
+                                     st["total_correspondences"]], dtype=np.float64),
+              "aligned_xyz": np.ascontiguousarray(cloud[:, 0:3], dtype=np.float32)}
+    if with_normals:
+        arrays["aligned_normals"] = np.ascontiguousarray(cloud[:, 4:7], dtype=np.float32)
+    if n > DUMP_ROWS:
+        arrays["aligned_rows"] = rows.numpy().astype(np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), a)
+
+
 def _protect_stdout():
     """Keep stdout for the ONE JSON line: libraries (NCCL prints its version banner) get stderr instead."""
     sys.stdout.flush()
@@ -728,7 +756,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-pipeline", action="store_true", help="e2e leg: one align in flight instead of two")
     ap.add_argument("--no-clocks", action="store_true", help="debug: do not sample clocks during the timed region")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (transformation, ICP state, aligned cloud) as DIR/*.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.steps < 1):
+        ap.error("--dump-outputs needs --impl ours and --steps >= 1 (the reference arm sizes its sample by timing)")
     if args.impl == "reference":
         run_reference(args)
     else:
